@@ -3,12 +3,10 @@
 MEASUREMENT INFRASTRUCTURE ONLY -- never imported by the product package (council_gan_b200).
 
 Where the reference comes from, in this order (SURVEY.md section 8c/8d):
-  1. ``$COUNCIL_REF_DIR``
-  2. ``/root/reference``                 (the build container)
-  3. ``<repo>/baseline/_ref``            (git-ignored install made by ``baseline/install_reference.py`` in the build
-                                          container; it travels to the GPU box with the snapshot, like a pip --target
-                                          install would)
-If none exists, callers fall back to the oracle port (oracle/council_oracle.py: a plain-PyTorch restatement that
+  1. ``$COUNCIL_REF_DIR``                (a checkout of Onr/Council-GAN)
+  2. ``<repo>/oracle/_ref``              (git-ignored install made by ``oracle/install_reference.py`` during the build; it
+                                          travels with a copy of the built tree, like a pip --target install would)
+If neither exists, callers fall back to the oracle port (oracle/council_oracle.py: a plain-PyTorch restatement that
 is pinned against the reference's own outputs) and say so (``kind: "port"``).
 
 Two ways of running it:
@@ -35,7 +33,7 @@ NEEDED = ('trainer_council.py', 'networks.py', 'utils.py', 'data.py')
 def find_reference():
     if os.environ.get('COUNCIL_REF_DISABLE') == '1':  # tests: exercise the oracle-port fallback
         return None
-    for p in (os.environ.get('COUNCIL_REF_DIR'), '/root/reference', os.path.join(HERE, '_ref')):
+    for p in (os.environ.get('COUNCIL_REF_DIR'), os.path.join(ROOT, 'oracle', '_ref')):
         if p and all(os.path.exists(os.path.join(p, f)) for f in NEEDED):
             return p
     return None
@@ -81,7 +79,7 @@ def make_step(trainer, hp, x_a, x_b, iteration):
 def build_reference_trainer(hp, device, ref_dir=None):
     ref_dir = ref_dir or find_reference()
     if ref_dir is None:
-        raise FileNotFoundError('no reference tree (COUNCIL_REF_DIR, /root/reference, baseline/_ref)')
+        raise FileNotFoundError('no reference tree (COUNCIL_REF_DIR, oracle/_ref)')
     cls = import_reference(ref_dir, cpu_shim=(str(device) == 'cpu'))
     seed_like_train_py(hp.get('random_seed', 1))
     tr = cls(hp, str(device))

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- training images/sec of the Council-GAN step (dis_update + dis_council_update + gen_update).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one full training iteration (train.py:241-250 order) over one synthetic minibatch.
@@ -13,8 +13,11 @@ the public Council_Trainer API with HOST (pinned) image tensors: H2D copies and 
 the timed region.  `roofline` is for the dominant convolution kernel, timed live with CUDA events on the
 launching stream in a second timed region of the same K steps (the headline region carries no per-kernel events).
 
+`--dump-outputs DIR` writes what the last step of the headline region handed its caller (see dump_outputs) as DIR/<name>.npy;
+inputs, initial weights and noise are seeded, so two builds run with the same arguments can be compared output for output.
+
 Comparison legs (measurement infrastructure, baseline/ref_runner.py):
-  * `cpu_baseline` / `--impl reference`: the UNMODIFIED reference (`$COUNCIL_REF_DIR` -> /root/reference -> baseline/_ref; else the
+  * `cpu_baseline` / `--impl reference`: the UNMODIFIED reference (`$COUNCIL_REF_DIR` -> oracle/_ref; else the
     oracle port, `kind: "port"`) on the host cores, on a bounded sample of the workload (batch 1 -- the batch really run is
     printed), with the thread count chosen by a sweep at THIS workload (host core count printed);
   * `gpu_library_baseline` (and `--impl reference-gpu`): the same unmodified reference on the same B200 under stock
@@ -201,6 +204,35 @@ def parity_check(trainer_cls, workload, dev, tc):
     return {'checked': True, 'case': case, 'worst_rel_loss_err_vs_reference': worst, 'tol': 1e-3, 'ok': bool(worst < 1e-3)}
 
 
+DUMP_SAMPLE = 1 << 20  # parameter values kept per network family (4 MB of float32): a few families stay far below 64 MB
+
+
+def dump_outputs(trainer, out_dir):
+    """Write what a caller of the step receives after it, as float32 DIR/<name>.npy: the per-member total losses the three
+    updates publish, and per network family (gen/dis/dis_council x direction) every member's updated state_dict, flattened
+    in key order and concatenated over the members.  A family larger than DUMP_SAMPLE values keeps a fixed, seeded sample
+    of them (same positions, in increasing order, on every run of the same workload)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    for name in ('loss_dis_total', 'loss_dis_council_total', 'loss_gen_total'):
+        vals = getattr(trainer, name + '_s', None)
+        if vals is not None:
+            arrays[name] = np.array([float(v) for v in vals], dtype=np.float32)
+    for d in ('a2b', 'b2a'):
+        for fam in ('gen', 'dis', 'dis_council'):
+            members = getattr(trainer, '%s_%s_s' % (fam, d), None)
+            if not members:
+                continue
+            # a generator's state_dict mixes device parameters with host-side norm running statistics
+            flat = torch.cat([v.detach().to('cpu', torch.float32).reshape(-1) for m in members for v in m.state_dict().values()]).numpy()
+            if flat.size > DUMP_SAMPLE:
+                flat = flat[np.sort(np.random.default_rng(0).choice(flat.size, DUMP_SAMPLE, replace=False))]
+            arrays['params_%s_%s' % (fam, d)] = flat
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -212,6 +244,7 @@ def main():
     ap.add_argument('--no-gpu-baseline', action='store_true')
     ap.add_argument('--no-parity-check', action='store_true')
     ap.add_argument('--tc', type=int, default=1, help='0: SIMT fp32 kernels only, 1: tcgen05 TF32 where supported')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
     assert args.warmup >= 0 and args.steps >= 1
     rank = int(os.environ.get('RANK', '0'))
@@ -317,6 +350,8 @@ def main():
     l0 = ops.launch_count()
     ms = timed(lambda: step(xa_d, xb_d), args.steps)   # the headline timed region: nothing but the step's own launches in the stream
     launches = ops.launch_count() - l0
+    if args.dump_outputs and rank == 0:  # the regions below keep training the same trainer
+        dump_outputs(trainer, args.dump_outputs)
     # second timed region of the same K steps with a CUDA-event pair around every convolution / HBM-pass launch (per-kernel averages for
     # the roofline): ~800 event records per step cost host time (the 128x128 configuration is launch-bound) and sit between kernels that
     # would otherwise overlap their launch, so they are kept out of the headline region; shares are taken against THIS region's time
@@ -436,7 +471,7 @@ def main():
         sys.path.insert(0, os.path.join(ROOT, 'baseline'))
         import ref_runner as rr
         try:
-            gb = rr.gpu_library_baseline(hp, xa_h, xb_h, it, dev, steps=10, warmup=3)
+            gb = rr.gpu_library_baseline(hp, xa_h, xb_h, it, dev, steps=args.steps, warmup=args.warmup)
             gb['ours_over_baseline'] = value / gb['value']
             gb['ours_over_baseline_cudnn_benchmark'] = value / gb['value_cudnn_benchmark'] if gb.get('value_cudnn_benchmark') else None
         except Exception as e:  # the comparison leg must never take the product line down

@@ -46,6 +46,40 @@ def test_reference_arm_other_ranks_exit_without_work():
     assert r.returncode == 0 and r.stdout.strip() == ''
 
 
+def test_dump_outputs_after_one_step(tmp_path):
+    """--dump-outputs: float32 arrays of the published losses and a fixed sample of the updated parameters, at most 64 MB."""
+    import numpy as np
+    import torch
+    import bench
+    from council_gan_b200.trainer_council import Council_Trainer
+    from ops_torch import TorchOps
+    hp, n, b, size, it = bench.load_hp('tiny_64_n2_b2')
+    torch.manual_seed(1)
+    tr = Council_Trainer(hp, 'cpu', _ops=TorchOps('cpu'))
+    xa, xb = bench.synth(b, size, 123)
+    bench.dump_outputs(tr, str(tmp_path / 'pre'))
+    tr.dis_update(xa, xb, hp)
+    tr.dis_council_update(xa, xb, hp)
+    tr.gen_update(xa, xb, hp, it)
+    for out in ('a', 'b'):
+        bench.dump_outputs(tr, str(tmp_path / out))
+    names = sorted(os.listdir(tmp_path / 'a'))
+    assert names == ['loss_dis_council_total.npy', 'loss_dis_total.npy', 'loss_gen_total.npy', 'params_dis_a2b.npy',
+                     'params_dis_council_a2b.npy', 'params_gen_a2b.npy']
+    assert sum(os.path.getsize(tmp_path / 'a' / f) for f in names) <= 64 << 20
+    for f in names:
+        a = np.load(tmp_path / 'a' / f)
+        assert a.dtype == np.float32 and np.isfinite(a).all() and np.array_equal(a, np.load(tmp_path / 'b' / f)), f
+    assert np.array_equal(np.load(tmp_path / 'a' / 'loss_gen_total.npy'), np.array([float(v) for v in tr.loss_gen_total_s], np.float32))
+    for fam in ('gen', 'dis', 'dis_council'):  # the dump holds the parameters after the step, not before it
+        f = 'params_%s_a2b.npy' % fam
+        assert not np.array_equal(np.load(tmp_path / 'a' / f), np.load(tmp_path / 'pre' / f)), f
+    # the documented sample: the generators' state_dicts in key order, concatenated over the members, at seeded sorted positions
+    full = torch.cat([v.detach().float().reshape(-1) for m in tr.gen_a2b_s for v in m.state_dict().values()]).numpy()
+    idx = np.sort(np.random.default_rng(0).choice(full.size, bench.DUMP_SAMPLE, replace=False))
+    assert np.array_equal(np.load(tmp_path / 'a' / 'params_gen_a2b.npy'), full[idx])
+
+
 def test_product_arm_needs_cuda():
     import torch
     if torch.cuda.is_available():

@@ -259,3 +259,40 @@ def test_batched_sample_on_gpu_matches_oracle_decode():
             assert (out[3][r].cpu() - o2[0]).abs().mean().item() < 5e-4
             assert torch.equal(out[0][r].cpu(), x_a[i])
     tr.ops.set_tensor_core_mode(1)
+
+
+def test_bench_dump_outputs_is_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs on the device: what it writes equals the state after its warm-up and timed steps, replayed here
+    with bench.py's seeds (the regions timed after the headline one keep training and must not leak into the dump)."""
+    import json
+    import os
+    import random
+    import subprocess
+    import sys
+    import numpy as np
+    import bench
+    from council_gan_b200 import Council_Trainer
+    warmup, steps = 1, 2
+    r = subprocess.run([sys.executable, os.path.join(bench.ROOT, 'bench.py'), '--workload', 'tiny_64_n2_b2', '--steps', str(steps),
+                        '--warmup', str(warmup), '--no-cpu-baseline', '--no-gpu-baseline', '--no-parity-check',
+                        '--dump-outputs', str(tmp_path)], capture_output=True, text=True, timeout=600, cwd=bench.ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])['steps'] == steps
+    hp, n, b, size, it = bench.load_hp('tiny_64_n2_b2')
+    random.seed(1)
+    np.random.seed(1)
+    torch.manual_seed(1)
+    tr = Council_Trainer(hp, 'cuda:0')
+    tr.ops.set_tensor_core_mode(1)
+    xa, xb = (t.to('cuda:0') for t in bench.synth(b, size, 123))
+    for _ in range(warmup + steps):
+        tr.dis_update(xa, xb, hp)
+        tr.dis_council_update(xa, xb, hp)
+        tr.gen_update(xa, xb, hp, it)
+        tr.update_learning_rate()
+    want = tmp_path / 'replay'
+    bench.dump_outputs(tr, str(want))
+    assert sorted(os.listdir(want)) == sorted(f for f in os.listdir(tmp_path) if f.endswith('.npy'))
+    for f in os.listdir(want):
+        got, ref = np.load(tmp_path / f), np.load(want / f)
+        assert got.shape == ref.shape and np.allclose(got, ref, rtol=1e-5, atol=1e-7), (f, float(np.abs(got - ref).max()))
